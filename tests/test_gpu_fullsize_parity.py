@@ -41,7 +41,7 @@ def _golden(name):
 
 def _bench_rhs(n):
     b = rhs_slab(0, n)
-    b /= np.sqrt(float(np.dot(b, b)))
+    b /= np.sqrt(float(np.sum(b * b)))      # fixed summation order: np.dot's depends on the host's BLAS thread count
     return b
 
 
