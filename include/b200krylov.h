@@ -32,6 +32,8 @@ extern "C" {
 #define B200_API __attribute__((visibility("default")))
 
 enum { B200_F64 = 0, B200_F32 = 1 };
+/* storage the SpMV of an operator streams (b200_csr_format) */
+enum { B200_FORMAT_CSR = 0, B200_FORMAT_DIA = 1 };
 
 enum {
   B200_OK = 0,
@@ -113,6 +115,9 @@ B200_API int b200_ctx_profile_enable(b200_ctx *ctx, int on);
 B200_API int b200_ctx_profile_read(b200_ctx *ctx, int slot, double *total_ms, int64_t *launches, int reset);
 /* Tuning knobs (do not change results beyond floating-point summation order):
  *   "spmv_kernel": 0 = auto, 1 = sub-warp-per-row kernel, 2 = TMA-streamed kernel (when the tiles fit)
+ *   "spmv_format": 0 (default) = operators that carry an offset-diagonal copy (b200_csr_format) stream it in the SpMV
+ *           of mul!, cg! and minres! (bitwise the same results as the CSR: same row sums, same order); 1 = always the
+ *           CSR.  Read at every launch, so one process can compare both on the same operator.
  *   "snake": 1 (default) = consecutive hot kernels of a solver sweep the rows in alternating directions so
  *           that each starts on the data the previous one touched last (L2 reuse); 0 = always ascending
  *   "orth_fused": 1 (default) = orthogonalize_and_normalize! (CGS / DGKS) is ONE cooperative launch (dots, update, norm,
@@ -171,6 +176,12 @@ B200_API int b200_csr_destroy(b200_csr *A);
 /* size(A,1) local, size(A,2) global, nnz local, eltype */
 B200_API int b200_csr_info(const b200_csr *A, int64_t *m_local, int64_t *n_global, int64_t *nnz_local, int *dtype,
                            int64_t *row_begin, int64_t *n_halo);
+/* Storage of the operator's SpMV under spmv_format 0.  Square single-GPU operators whose nonzeros lie on at most 8
+ * diagonals (col - row offsets), and whose offset-diagonal (DIA) copy -- one value array per diagonal and a presence
+ * byte per row -- is at most 0.8x the CSR bytes, get that copy at construction: *format = B200_FORMAT_DIA, *ndiag the
+ * number of diagonals and offsets[0..ndiag) (room for 8) the ascending offsets.  Otherwise B200_FORMAT_CSR, ndiag 0.
+ * Any output pointer may be NULL. */
+B200_API int b200_csr_format(const b200_csr *A, int *format, int *ndiag, int64_t *offsets);
 /* adjoint(A) as an operator (reference: `adjoint(A)` stored by LanczosDecomp src/qmr.jl:54 and used by
  * mul!(y, A', x) at src/qmr.jl:76, src/lsqr.jl:132,172, src/lsmr.jl:118,172).  Built on the device from the CSR of A
  * (real element types: adjoint == transpose).  Single-GPU contexts; on multi-GPU contexts pass the row slabs of A'

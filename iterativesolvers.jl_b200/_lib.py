@@ -148,6 +148,7 @@ SIGNATURES = {
     "b200_csr_info": (_INT, [_P, C.POINTER(_I64), C.POINTER(_I64), C.POINTER(_I64), C.POINTER(_INT),
                              C.POINTER(_I64), C.POINTER(_I64)]),
     "b200_csr_transpose": (_INT, [_P, _P, C.POINTER(_P)]),
+    "b200_csr_format": (_INT, [_P, C.POINTER(_INT), C.POINTER(_INT), C.POINTER(_I64)]),
     "b200_csr_diag": (_INT, [_P, _P, _P]),
     "b200_csr_download": (_INT, [_P, _P, _P, _P, _P]),
     "b200_halo_plan_create": (_INT, [_INT, _INT, C.POINTER(_I64), C.POINTER(_P)]),

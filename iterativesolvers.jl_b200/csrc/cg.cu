@@ -25,7 +25,7 @@
 #include <cooperative_groups.h>
 
 #include "blas1.cuh"
-#include "spmv_stream.cuh"
+#include "spmv_dia.cuh"
 #include "linop.cuh"
 
 using namespace b200;
@@ -278,6 +278,25 @@ __global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm)
   wait_halo(cm);
   CgDotEpi<T> epi{c, xv.x, 0.0};
   spmv_stream_tiles<T, LPR>(rowptr, colind, vals, xv, m, epi, reinterpret_cast<StreamSmem<T> *>(smem_raw), cm.rev != 0);
+  pdl_launch_dependents();
+  const double acc = block_sum<kStreamThreads>(epi.acc, red);
+  double total;
+  if (grid_reduce_finish<kStreamThreads>(acc, partials, ticket, red, &total) && threadIdx.x < 32)
+    cg_finish(FIN_DOT, s, total, nullptr, cm);
+}
+
+// K2 on the DIA copy (spmv_dia.cuh): same row -> thread -> CTA mapping and row sums as the CSR stream, so c and <u,c>
+// are bitwise the same
+template <typename T>
+__global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm)
+    k_cg_spmv_dot_dia(DiaView<T> dv, XView<T> xv, int64_t m, T *__restrict__ c, CgScal *s, double *partials,
+                      unsigned int *ticket, Comm cm) {
+  pdl_wait();
+  if (s->done) return;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  __shared__ double red[kStreamThreads / 32];
+  CgDotEpi<T> epi{c, xv.x, 0.0};
+  spmv_dia_tiles<T>(dv, xv, m, epi, reinterpret_cast<DiaSmem<T> *>(smem_raw), cm.rev != 0);
   pdl_launch_dependents();
   const double acc = block_sum<kStreamThreads>(epi.acc, red);
   double total;
@@ -548,7 +567,14 @@ struct CgEngine {
     }
     XView<T> xv = make_xview<T>(A, u, peer && !fold_halo);
     const Comm cm = comm(!fold_halo, next_sweep());
-    if (use_stream(ctx, A)) {
+    if (use_dia(ctx, A)) {
+      const int grid = stream_grid_size(ctx, A);
+      const size_t smem = sizeof(DiaSmem<T>);
+      ProfScope prof(ctx, 0);
+      B200_SMEM_ATTR_ONCE(ctx, smem, k_cg_spmv_dot_dia<T>);
+      B200_CUDA(launch_chained(ctx->opt_pdl != 0, k_cg_spmv_dot_dia<T>, dim3(grid), dim3(kStreamThreads), smem,
+                               ctx->stream, make_diaview<T>(A), xv, n, c, s, ctx->red.partials, ctx->red.ticket, cm));
+    } else if (use_stream(ctx, A)) {
       const int grid = stream_grid_size(ctx, A);
       const size_t smem = sizeof(StreamSmem<T>);
       ProfScope prof(ctx, 0);

@@ -97,6 +97,7 @@ struct b200_ctx {
   double *h_scalars = nullptr;   // pinned host mirror (64 doubles)
   int *h_flags = nullptr;        // pinned host flags (16 ints)
   int opt_spmv_kernel = 0;       // b200_ctx_set_option("spmv_kernel"): 0 auto, 1 sub-warp per row, 2 TMA stream
+  int opt_spmv_format = 0;       // b200_ctx_set_option("spmv_format"): 0 auto (the DIA copy when the operator has one), 1 CSR
   int opt_comm = 0;              // b200_ctx_set_option("comm"): 0 auto (peer memory if mapped), 1 NCCL, 2 peer memory
   int opt_lobpcg_mma = 1;        // b200_ctx_set_option("lobpcg_mma"): fp32 LOBPCG blocks on the tensor cores (3xTF32): 1 = Rayleigh-Ritz Gram on
                                  // tcgen05 (TMEM accumulators), 2 = legacy mma.sync Gram, 0 = SIMT kernels

@@ -1,6 +1,7 @@
 // csr.cu -- building the device operator: SparseMatrixCSC -> CSR int32 (device transpose),
 // CSR row slabs, the on-device laplace_matrix generator, halo plans and the halo exchange.
 #include <algorithm>
+#include <climits>
 #include <cub/cub.cuh>
 
 #include "csr.cuh"
@@ -322,6 +323,81 @@ __global__ void k_tile_max(const int *__restrict__ rowptr, int64_t m, int R, int
   if ((threadIdx.x & 31) == 0) atomicMax(out, local);
 }
 
+// DIA detection, pass 1 (one read of rowptr/colind): the set of distinct col - row offsets, at most kDiaMaxDiags of
+// them, and whether every row's columns are strictly ascending.  Each block collects its offsets in a shared set
+// (insertion by CAS into the first free slot: no value lands in two slots) and merges it into the global set the same
+// way.  flags[0]: more than kDiaMaxDiags offsets; flags[1]: a row with unsorted or repeated columns.
+constexpr int kDiaEmpty = INT_MIN;   // col - row of two int32 indices in [0, 2^31) is > INT_MIN
+__device__ __forceinline__ bool dia_set_insert(int *set, int v) {
+  for (int s = 0; s < kDiaMaxDiags; ++s) {
+    const int cur = *(volatile int *)&set[s];
+    if (cur == v) return true;
+    if (cur == kDiaEmpty) {
+      const int old = atomicCAS(&set[s], kDiaEmpty, v);
+      if (old == kDiaEmpty || old == v) return true;
+    }
+  }
+  return false;
+}
+__global__ void k_dia_scan(const int *__restrict__ rowptr, const int *__restrict__ colind, int64_t m,
+                           int *__restrict__ gset, int *__restrict__ flags) {
+  __shared__ int set[kDiaMaxDiags];
+  __shared__ int bad[2];
+  if (threadIdx.x < kDiaMaxDiags) set[threadIdx.x] = kDiaEmpty;
+  if (threadIdx.x < 2) bad[threadIdx.x] = 0;
+  __syncthreads();
+  int last = kDiaEmpty;   // this thread's last inserted offset (rows of a stencil repeat the same few)
+  bool over = false, unsorted = false;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < m && !over; i += (int64_t)gridDim.x * blockDim.x) {
+    const int b = rowptr[i], e = rowptr[i + 1];
+    int prev = -1;
+    for (int k = b; k < e; ++k) {
+      const int c = colind[k];
+      unsorted |= c <= prev;
+      prev = c;
+      const int v = c - (int)i;
+      if (v != last && !dia_set_insert(set, v)) {
+        over = true;
+        break;
+      }
+      last = v;
+    }
+  }
+  if (over) bad[0] = 1;
+  if (unsorted) bad[1] = 1;
+  __syncthreads();
+  if (threadIdx.x < kDiaMaxDiags && set[threadIdx.x] != kDiaEmpty && !dia_set_insert(gset, set[threadIdx.x]))
+    flags[0] = 1;
+  if (threadIdx.x < 2 && bad[threadIdx.x]) flags[threadIdx.x] = 1;
+}
+
+// DIA pass 2 (one read of the CSR): scatter the values, set the presence bits.  flags[2]: an offset outside the set
+// or a bit set twice (cannot happen after a clean pass 1; checked so that a DIA copy is never wrong).
+struct DiaOffsets {
+  int off[kDiaMaxDiags];
+  int ndiag;
+};
+template <typename T>
+__global__ void k_dia_fill(const int *__restrict__ rowptr, const int *__restrict__ colind, const T *__restrict__ vals,
+                           int64_t m, DiaOffsets o, int64_t ld, T *__restrict__ dvals, uint8_t *__restrict__ dmask,
+                           int *__restrict__ flags) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < m; i += (int64_t)gridDim.x * blockDim.x) {
+    unsigned int bits = 0;
+    for (int k = rowptr[i]; k < rowptr[i + 1]; ++k) {
+      const int v = colind[k] - (int)i;
+      int d = 0;
+      while (d < o.ndiag && o.off[d] != v) ++d;
+      if (d == o.ndiag || ((bits >> d) & 1u)) {
+        flags[2] = 1;
+        continue;
+      }
+      bits |= 1u << d;
+      dvals[d * ld + i] = vals[k];
+    }
+    dmask[i] = (uint8_t)bits;
+  }
+}
+
 template <typename T>
 __global__ void k_pack(const int *__restrict__ idx, const T *__restrict__ x, int64_t n, T *__restrict__ out) {
   for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x)
@@ -333,6 +409,86 @@ int grid_for(const b200_ctx *ctx, int64_t n, int threads = 256) {
   int64_t cap = (int64_t)ctx->sm_count * 8;
   if (g < 1) g = 1;
   return (int)(g < cap ? g : cap);
+}
+
+void free_dia(b200_csr *A) {
+  cudaFree(A->dia_vals);
+  cudaFree(A->dia_mask);
+  A->dia_vals = nullptr;
+  A->dia_mask = nullptr;
+  A->dia_ndiag = 0;
+  A->dia_m_pad = 0;
+}
+
+// Builds the DIA copy of a square single-GPU operator whose nonzeros lie on at most kDiaMaxDiags diagonals, when that
+// copy is at most 0.8x the CSR bytes.  Not building it is never an error: a failed allocation leaves the CSR alone.
+int build_dia(b200_ctx *ctx, b200_csr *A) {
+  const int64_t m = A->m_local;
+  if (ctx->world != 1 || A->n_halo != 0 || !is_square(A) || m == 0 || A->nnz == 0 || A->stream_lpr != 1) return B200_OK;
+  cudaStream_t st = ctx->stream;
+  int *d_buf = nullptr;   // [0, 8): offset set, [8, 11): flags
+  B200_CUDA(cudaMalloc(&d_buf, sizeof(int) * 16));
+  std::vector<int> h_init(16, 0);
+  for (int s = 0; s < kDiaMaxDiags; ++s) h_init[s] = kDiaEmpty;
+  auto done = [&](int s) {
+    cudaFree(d_buf);
+    return s;
+  };
+#define CK(call)                                                                        \
+  do {                                                                                  \
+    cudaError_t _e = (call);                                                            \
+    if (_e != cudaSuccess) {                                                            \
+      set_error("%s:%d %s in `%s`", __FILE__, __LINE__, cudaGetErrorString(_e), #call); \
+      free_dia(A);                                                                      \
+      return done(B200_ERR_CUDA);                                                       \
+    }                                                                                   \
+  } while (0)
+  CK(cudaMemcpyAsync(d_buf, h_init.data(), sizeof(int) * 16, cudaMemcpyHostToDevice, st));
+  k_dia_scan<<<grid_for(ctx, m), 256, 0, st>>>(A->rowptr, A->colind, m, d_buf, d_buf + kDiaMaxDiags);
+  ctx->launches++;
+  CK(cudaMemcpyAsync(ctx->h_flags, d_buf, sizeof(int) * 16, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+  if (ctx->h_flags[kDiaMaxDiags] || ctx->h_flags[kDiaMaxDiags + 1]) return done(B200_OK);
+  std::vector<int> offs;
+  for (int s = 0; s < kDiaMaxDiags; ++s)
+    if (ctx->h_flags[s] != kDiaEmpty) offs.push_back(ctx->h_flags[s]);
+  std::sort(offs.begin(), offs.end());
+  const int nd = (int)offs.size();
+  const size_t vs = dtype_size(A->dtype);
+  const double dia_bytes = (double)nd * (double)m * (double)vs + (double)m;
+  const double csr_bytes = (double)A->nnz * (double)(vs + 4) + 4.0 * (double)(m + 1);
+  if (nd == 0 || dia_bytes > 0.8 * csr_bytes) return done(B200_OK);
+  const int64_t m_pad = (m + kDiaRowAlign - 1) / kDiaRowAlign * kDiaRowAlign;
+  if (cudaMalloc(&A->dia_vals, vs * nd * m_pad) != cudaSuccess || cudaMalloc(&A->dia_mask, m_pad) != cudaSuccess) {
+    cudaGetLastError();   // out of memory is not sticky: clear it and keep serving the CSR
+    free_dia(A);
+    return done(B200_OK);
+  }
+  CK(cudaMemsetAsync(A->dia_vals, 0, vs * nd * m_pad, st));
+  CK(cudaMemsetAsync(A->dia_mask, 0, m_pad, st));
+  DiaOffsets o;
+  o.ndiag = nd;
+  for (int d = 0; d < kDiaMaxDiags; ++d) o.off[d] = d < nd ? offs[d] : 0;
+  if (A->dtype == B200_F64)
+    k_dia_fill<double><<<grid_for(ctx, m), 256, 0, st>>>(A->rowptr, A->colind, (const double *)A->vals, m, o, m_pad,
+                                                          (double *)A->dia_vals, A->dia_mask, d_buf + kDiaMaxDiags);
+  else
+    k_dia_fill<float><<<grid_for(ctx, m), 256, 0, st>>>(A->rowptr, A->colind, (const float *)A->vals, m, o, m_pad,
+                                                         (float *)A->dia_vals, A->dia_mask, d_buf + kDiaMaxDiags);
+  ctx->launches++;
+  CK(cudaMemcpyAsync(ctx->h_flags, d_buf + kDiaMaxDiags, sizeof(int) * 3, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  CK(cudaGetLastError());
+#undef CK
+  if (ctx->h_flags[2]) {
+    free_dia(A);
+    return done(B200_OK);
+  }
+  A->dia_ndiag = nd;
+  A->dia_m_pad = m_pad;
+  for (int d = 0; d < kDiaMaxDiags; ++d) A->dia_off[d] = d < nd ? offs[d] : 0;
+  return done(B200_OK);
 }
 
 int finish_operator(b200_ctx *ctx, b200_csr *A, const b200_halo_plan *plan) {
@@ -363,6 +519,7 @@ int finish_operator(b200_ctx *ctx, b200_csr *A, const b200_halo_plan *plan) {
         break;
       }
   }
+  B200_TRY(build_dia(ctx, A));
   B200_CUDA(cudaMemsetAsync(d_max, 0, sizeof(double) * 8, ctx->stream));
   // halo exchange lists
   const int W = ctx->world;
@@ -761,6 +918,8 @@ int b200_csr_destroy(b200_csr *A) {
   cudaFree(A->send_idx);
   cudaFree(A->send_buf);
   cudaFree(A->halo);
+  cudaFree(A->dia_vals);
+  cudaFree(A->dia_mask);
   if (A->st_plan && A->st_plan_free) A->st_plan_free(A->st_plan);
   delete A;
   return B200_OK;
@@ -775,6 +934,15 @@ int b200_csr_info(const b200_csr *A, int64_t *m_local, int64_t *n_global, int64_
   if (dtype) *dtype = A->dtype;
   if (row_begin) *row_begin = A->row_begin;
   if (n_halo) *n_halo = A->n_halo;
+  return B200_OK;
+}
+
+int b200_csr_format(const b200_csr *A, int *format, int *ndiag, int64_t *offsets) {
+  B200_REQUIRE(A, "A is NULL");
+  if (format) *format = A->dia_ndiag > 0 ? B200_FORMAT_DIA : B200_FORMAT_CSR;
+  if (ndiag) *ndiag = A->dia_ndiag;
+  if (offsets)
+    for (int d = 0; d < A->dia_ndiag; ++d) offsets[d] = A->dia_off[d];
   return B200_OK;
 }
 

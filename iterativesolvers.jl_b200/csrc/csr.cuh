@@ -17,6 +17,10 @@ namespace b200 {
 // inside the allocations (spmv_stream.cuh)
 constexpr int64_t kRowptrPad = 520;
 constexpr int64_t kNnzPad = 16;
+// offset-diagonal (DIA) copy of a square single-GPU operator whose nonzeros lie on at most this many diagonals
+// (spmv_dia.cuh); rows are padded to whole 512-row tiles so that every bulk copy of a tile stays in bounds
+constexpr int kDiaMaxDiags = 8;
+constexpr int64_t kDiaRowAlign = 512;
 }  // namespace b200
 using b200::kNnzPad;
 using b200::kRowptrPad;
@@ -32,6 +36,14 @@ struct b200_csr {
   void *vals = nullptr;    // nnz
   int max_row_nnz = 0;
   double avg_row_nnz = 0.0;
+  // DIA copy (spmv_dia.cuh), built next to the CSR when the operator has few distinct col - row offsets:
+  // dia_vals[d * dia_m_pad + row] = A[row, row + dia_off[d]], bit d of dia_mask[row] set iff the CSR row stores that
+  // entry (explicit zeros included).  Offsets ascending = column order.  dia_ndiag == 0: no DIA copy.
+  int dia_ndiag = 0;
+  int64_t dia_off[b200::kDiaMaxDiags] = {0};
+  int64_t dia_m_pad = 0;       // m_local rounded up to kDiaRowAlign
+  void *dia_vals = nullptr;    // dia_ndiag * dia_m_pad values, diagonal-major
+  uint8_t *dia_mask = nullptr; // dia_m_pad bytes (zero in the padding rows)
   // halo exchange state (world > 1)
   std::vector<int64_t> send_count, send_offset, recv_count, recv_offset;  // per peer
   int64_t n_send = 0;

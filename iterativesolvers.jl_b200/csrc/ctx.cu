@@ -245,6 +245,11 @@ int b200_ctx_set_option(b200_ctx *c, const char *name, int64_t value) {
     c->opt_spmv_kernel = (int)value;
     return B200_OK;
   }
+  if (strcmp(name, "spmv_format") == 0) {
+    B200_REQUIRE(value == 0 || value == 1, "spmv_format must be 0 (auto) or 1 (CSR)");
+    c->opt_spmv_format = (int)value;
+    return B200_OK;
+  }
   if (strcmp(name, "snake") == 0) {
     c->opt_snake = value != 0;
     return B200_OK;
@@ -282,6 +287,7 @@ int b200_ctx_set_option(b200_ctx *c, const char *name, int64_t value) {
 int b200_ctx_get_option(const b200_ctx *c, const char *name, int64_t *value) {
   B200_REQUIRE(c && name && value, "NULL argument");
   if (strcmp(name, "spmv_kernel") == 0) *value = c->opt_spmv_kernel;
+  else if (strcmp(name, "spmv_format") == 0) *value = c->opt_spmv_format;
   else if (strcmp(name, "comm") == 0) *value = c->opt_comm;
   else if (strcmp(name, "lobpcg_mma") == 0) *value = c->opt_lobpcg_mma;
   else if (strcmp(name, "snake") == 0) *value = c->opt_snake;

@@ -8,7 +8,7 @@
 // The vector "rotation" of :147-148 is a pointer swap done by the host (it is unconditional).
 // Algorithmic bytes per iteration: nnz*(V+4) + (n+1)*4 + 14*n*V.
 #include "blas1.cuh"
-#include "spmv_stream.cuh"
+#include "spmv_dia.cuh"
 
 using namespace b200;
 
@@ -196,6 +196,22 @@ __global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm)
     mr_finish(MR_PROJ, m, total, nullptr, single);
 }
 
+// Ka on the DIA copy (spmv_dia.cuh): bitwise the result of k_mr_spmv_stream<T, 1>
+template <typename T>
+__global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm)
+    k_mr_spmv_dia(DiaView<T> dv, XView<T> xv, const T *__restrict__ v_prev, T *__restrict__ v_next, int64_t n,
+                  MrScal *m, double *partials, unsigned int *ticket, int single) {
+  if (m->done) return;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  __shared__ double red[kStreamThreads / 32];
+  MrEpi<T> epi{v_next, v_prev, xv.x, (T)m->H[1], m->iteration > 1, 0.0};
+  spmv_dia_tiles<T>(dv, xv, n, epi, reinterpret_cast<DiaSmem<T> *>(smem_raw));
+  const double acc = block_sum<kStreamThreads>(epi.acc, red);
+  double total;
+  if (grid_reduce_finish<kStreamThreads>(acc, partials, ticket, red, &total) && threadIdx.x == 0)
+    mr_finish(MR_PROJ, m, total, nullptr, single);
+}
+
 // Kb
 template <typename T>
 __global__ void __launch_bounds__(kThreads) k_mr_orth(const T *__restrict__ v_curr, T *__restrict__ v_next, int64_t n,
@@ -313,7 +329,14 @@ int minres_impl(b200_ctx *ctx, const b200_csr *A, T *x, const T *b, const b200_m
     for (int64_t it = 0; it < batch; ++it) {
       B200_TRY(halo_exchange(ctx, A, v_curr));
       XView<T> xv = make_xview<T>(A, v_curr);
-      if (use_stream(ctx, A)) {
+      if (use_dia(ctx, A)) {
+        const int grid = stream_grid_size(ctx, A);
+        const size_t smem = sizeof(DiaSmem<T>);
+        ProfScope prof(ctx, 0);
+        B200_SMEM_ATTR_ONCE(ctx, smem, k_mr_spmv_dia<T>);
+        k_mr_spmv_dia<T><<<grid, kStreamThreads, smem, st>>>(make_diaview<T>(A), xv, v_prev, v_next, n, m,
+                                                             ctx->red.partials, ctx->red.ticket, single);
+      } else if (use_stream(ctx, A)) {
         const int grid = stream_grid_size(ctx, A);
         const size_t smem = sizeof(StreamSmem<T>);
         ProfScope prof(ctx, 0);

@@ -1,5 +1,5 @@
 // spmv.cu -- mul!(y, A, x) and mul!(Y, A, X) (block SpMM) on the device CSR.
-#include "spmv_stream.cuh"
+#include "spmv_dia.cuh"
 
 using namespace b200;
 
@@ -81,6 +81,27 @@ __global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm)
   spmv_stream_tiles<T, LPR>(rowptr, colind, vals, xv, m, epi, reinterpret_cast<StreamSmem<T> *>(smem_raw));
 }
 
+// the same on the DIA copy (spmv_dia.cuh)
+template <typename T>
+__global__ void __launch_bounds__(kStreamThreads, kStreamCtasPerSm)
+    k_spmv_dia(DiaView<T> dv, XView<T> xv, int64_t m, T *__restrict__ y, const int *__restrict__ gate, int gate_mask) {
+  if (gate && (*gate & gate_mask)) return;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  StoreEpi<T> epi{y};
+  spmv_dia_tiles<T>(dv, xv, m, epi, reinterpret_cast<DiaSmem<T> *>(smem_raw));
+}
+
+template <typename T>
+int launch_spmv_dia(b200_ctx *ctx, const b200_csr *A, const void *x, void *y, const int *gate, int gate_mask) {
+  const int grid = stream_grid_size(ctx, A);
+  const size_t smem = sizeof(DiaSmem<T>);
+  B200_SMEM_ATTR_ONCE(ctx, smem, k_spmv_dia<T>);
+  k_spmv_dia<T><<<grid, kStreamThreads, smem, ctx->stream>>>(make_diaview<T>(A), make_xview<T>(A, x), A->m_local,
+                                                             (T *)y, gate, gate_mask);
+  B200_LAUNCH_CHECK(ctx);
+  return B200_OK;
+}
+
 template <typename T>
 int launch_spmv_stream(b200_ctx *ctx, const b200_csr *A, const void *x, void *y, const int *gate, int gate_mask) {
   XView<T> xv = make_xview<T>(A, x);
@@ -108,6 +129,7 @@ int launch_spmv_stream(b200_ctx *ctx, const b200_csr *A, const void *x, void *y,
 template <typename T>
 int launch_spmv(b200_ctx *ctx, const b200_csr *A, const void *x, void *y, const int *gate = nullptr, int gate_mask = 0) {
   if (A->m_local == 0) return B200_OK;
+  if (use_dia(ctx, A)) return launch_spmv_dia<T>(ctx, A, x, y, gate, gate_mask);
   if (use_stream(ctx, A)) return launch_spmv_stream<T>(ctx, A, x, y, gate, gate_mask);
   XView<T> xv = make_xview<T>(A, x);
   const int lpr = pick_lpr(A->avg_row_nnz);

@@ -227,6 +227,21 @@ class B200CSR:
         self.mul_(yd, xd)
         return yd.numpy()
 
+    @property
+    def format(self) -> str:
+        """"dia" if the SpMV streams the operator's offset-diagonal copy (spmv_format 0), else "csr"."""
+        fmt = C.c_int()
+        check(lib().b200_csr_format(self._h, C.byref(fmt), None, None))
+        return "dia" if fmt.value == 1 else "csr"
+
+    @property
+    def dia_offsets(self) -> list:
+        """the ascending col - row offsets of the DIA copy ([] for a CSR-only operator)."""
+        nd = C.c_int()
+        offs = (C.c_int64 * 8)()
+        check(lib().b200_csr_format(self._h, None, C.byref(nd), offs))
+        return [int(offs[d]) for d in range(nd.value)]
+
     def diag(self) -> DeviceArray:
         d = DeviceArray(self.ctx, self.m_local, self.dtype)
         check(lib().b200_csr_diag(self.ctx._h, self._h, d._p))

@@ -30,6 +30,8 @@ HOT = {
     "lobpcg_gram_legacy": ("k_gram_rr_tcILi2E", "LOBPCG Rayleigh-Ritz Gram products, legacy mma.sync path (kept for comparison)"),
     "pass_generic": ("k_passINS_8QmrWNextIdEE", "the fused-pass kernel of the general engines (one instantiation: QMR's w-recurrence pass)"),
     "spmv_stream_f64": ("k_spmv_streamIdLi8E", "mul!(y, A, x): TMA-bulk streamed CSR SpMV"),
+    "cg_k2_spmv_dot_dia_f64": ("k_cg_spmv_dot_diaIdE", "K2 of cg! on the offset-diagonal copy: TMA-bulk streamed values + row masks"),
+    "spmv_dia_f64": ("k_spmv_diaIdE", "mul!(y, A, x) on the offset-diagonal copy"),
 }
 KEY = re.compile(r"\b(UBLKCP|UTMALDG|UTMASTG|SYNCS|UTC[A-Z]*MMA|UTCBAR|UTCCP|LDTM|STTM|UTCALLOC|HMMA|DFMA|DADD|DMUL|FFMA|"
                  r"LDG|STG|LDS|STS|REDG|ATOMG|SHFL|BAR|ACQBULK|ELECT|LDGSTS|CCTL|MEMBAR|ERRBAR|FENCE)\b")
